@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json metric: RQ-VAE items/sec for the fused L-level quantiser (64K x 768, K=256, L=3).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (tokenise: L chained distance+argmin levels) over one batch of 65 536
 synthetic unit-norm item vectors per GPU.  Prints ONE JSON line (rank 0).  Under torchrun every rank tokenises its
@@ -25,6 +25,10 @@ own shard (items are independent: weak scaling, no data-path collective); the ti
 
 --impl reference times that CPU port as the reference arm (the reference is pure Python/PyTorch: there is nothing
 to compile into oracle/_ref, see DESIGN.md).
+
+--dump-outputs DIR writes what the last timed step returned -- the [65 536, L] semantic ids -- as DIR/ids.npy (float32,
+exact for ids < 2^24; DIR/ids_rank<r>.npy per rank under torchrun).  The inputs are seeded, so two builds (or the two
+--impl arms) run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -51,6 +55,14 @@ def make_problem(n_items, seed=1234):
     x = I.unit_rows(seed, n_items, D)
     _, cbs = I.rq_problem(8192, D, K, L, seed=seed, x=x[:8192])
     return x, cbs
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor or array; each is written as out_dir/<name>.npy in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def algorithmic_bytes(n_items):
@@ -172,11 +184,14 @@ def run_reference(args):
         OT.rq_tokenize(xt, cbt)
     t0 = time.perf_counter()
     best = float("inf")
+    ids = None
     for _ in range(args.steps):
         t1 = time.perf_counter()
-        OT.rq_tokenize(xt, cbt)
+        ids = OT.rq_tokenize(xt, cbt)
         best = min(best, time.perf_counter() - t1)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ids": ids})
     val = args.steps * sample / dt
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -435,6 +450,7 @@ def main():
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--path", default="auto", choices=["auto", "tc", "simt"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -609,6 +625,8 @@ def main():
         agree = float((ids[:512].cpu().numpy() == chk).all(1).mean())
         out["config"]["oracle_agreement_512"] = agree
         print(json.dumps(out))
+    if args.dump_outputs:                               # `ids` is still the last timed step's result
+        dump_outputs(args.dump_outputs, {"ids" if world == 1 else f"ids_rank{rank}": ids})
     if world > 1:
         dist.destroy_process_group()
 

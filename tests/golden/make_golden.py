@@ -69,9 +69,11 @@ def make_quantize(D, K, cb, mode, beta=BETA):
 
 # ------------------------------------------------------------------ G1: single-level Quantize, all modes, with grads
 def g_quantize():
+    """Full embeddings / input gradients are kept for the first `keep` rows only (the fixture stays under 1 MB); row sums
+    cover every row."""
     out = {}
-    for tag, (B, D, K, keep) in {"c1": (1024, 16, 32, 1024), "d32": (1024, 32, 256, 1024),
-                                 "d768": (512, 768, 256, 48)}.items():
+    for tag, (B, D, K, keep) in {"c1": (1024, 16, 32, 256), "d32": (1024, 32, 256, 128),
+                                 "d768": (512, 768, 256, 16)}.items():
         x, cbs = I.rq_problem(B, D, K, 1, seed=100 + D)
         cb = cbs[0]
         g_out = I.randn(200 + D, B, D)
@@ -86,6 +88,7 @@ def g_quantize():
         out[f"{tag}_eval_ids"] = o.ids.numpy().astype(np.int16)
         out[f"{tag}_eval_loss"] = o.loss.numpy()
         out[f"{tag}_eval_emb"] = o.embeddings.numpy()[:keep]
+        out[f"{tag}_eval_emb_rowsum"] = o.embeddings.double().sum(1).numpy()
         for mname, mode in MODES.items():
             q = make_quantize(D, K, cb, mode).train()
             xt = t(x).clone().requires_grad_(True)
@@ -98,6 +101,7 @@ def g_quantize():
             out[f"{tag}_{mname}_ids"] = o.ids.numpy().astype(np.int16)
             out[f"{tag}_{mname}_loss"] = o.loss.detach().numpy()
             out[f"{tag}_{mname}_emb"] = o.embeddings.detach().numpy()[:keep]
+            out[f"{tag}_{mname}_emb_rowsum"] = o.embeddings.detach().double().sum(1).numpy()
             out[f"{tag}_{mname}_gx"] = xt.grad.numpy()[:keep]
             out[f"{tag}_{mname}_gx_rowsum"] = xt.grad.double().sum(1).numpy()
             gc = q.embedding.weight.grad.numpy()
@@ -214,6 +218,7 @@ def g_beauty():
 
 # ------------------------------------------------------------------ G5: MLP + l2norm
 def g_mlp():
+    """gx is kept for the first 32 of the 256 rows (the fixture stays under 1 MB); its row sums cover every row."""
     dims = [768, 512, 256, 128, 32]
     ws = I.mlp_weights(500, dims)
     x = I.unit_rows(501, 256, 768)
@@ -228,7 +233,8 @@ def g_mlp():
         gy = I.randn(502, 256, 32)
         (y * t(gy)).sum().backward()
         out[f"y_norm{int(norm)}"] = y.detach().numpy()
-        out[f"gx_norm{int(norm)}"] = xt.grad.numpy()
+        out[f"gx_norm{int(norm)}"] = xt.grad.numpy()[:32]
+        out[f"gx_rowsum_norm{int(norm)}"] = xt.grad.double().sum(1).numpy()
         out[f"gw3_norm{int(norm)}"] = mlp.mlp[6].weight.grad.numpy()
         out[f"gw0_rowsum_norm{int(norm)}"] = mlp.mlp[0].weight.grad.double().sum(1).numpy()
     out["l2norm"] = ref.normalize.l2norm(t(x[:, :40] * 0.0 + I.randn(503, 256, 40))).numpy()
@@ -393,7 +399,44 @@ def g_beam():
     save("beam", **out)
 
 
+# ------------------------------------------------------------------ G9: what dropin.py must satisfy
+def g_dropin():
+    """Read from the unmodified tree: every `from modules.* / init.* / distributions.* import name` (file:module:name), the
+    RqVae / SemanticIdTokenizer calls (file:class:positional count:keywords), and the shipped Beauty checkpoint with its
+    tensor payloads zeroed -- the pickle (class paths, model_config, state-dict layout) is kept byte for byte, and the zeros
+    compress to a few KB."""
+    import ast
+    import io
+    import zipfile
+    root = ref_harness.REFERENCE
+    imports, calls = [], []
+    for dirpath, dirs, files in os.walk(root):
+        dirs.sort()
+        for f in sorted(files):
+            if not f.endswith(".py"):
+                continue
+            rel = os.path.relpath(os.path.join(dirpath, f), root)
+            with open(os.path.join(dirpath, f)) as fh:
+                tree = ast.parse(fh.read())
+            for node in ast.walk(tree):
+                if isinstance(node, ast.ImportFrom) and node.module and node.module.split(".")[0] in (
+                        "modules", "init", "distributions"):
+                    imports += [f"{rel}:{node.module}:{a.name}" for a in node.names]
+                elif isinstance(node, ast.Call) and getattr(node.func, "id", None) in ("RqVae", "SemanticIdTokenizer"):
+                    calls.append(f"{rel}:{node.func.id}:{len(node.args)}:" + ",".join(k.arg for k in node.keywords if k.arg))
+    buf = io.BytesIO()
+    path = os.path.join(root, "trained_models/rqvae_amazon_beauty/checkpoint_high_entropy.pt")
+    with zipfile.ZipFile(path) as src, zipfile.ZipFile(buf, "w", zipfile.ZIP_STORED) as dst:
+        for info in src.infolist():
+            data = src.read(info.filename)
+            if "/data/" in info.filename:                     # <archive>/data/<key>: one tensor storage each
+                data = bytes(len(data))
+            dst.writestr(info.filename, data)
+    save("dropin", imports=np.array(imports), calls=np.array(calls), checkpoint=np.frombuffer(buf.getvalue(), np.uint8))
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["quantize", "rqvae_c1", "rq_ns", "beauty", "mlp", "kmeans", "gumbel", "tokenizer", "beam"]
+    which = sys.argv[1:] or ["quantize", "rqvae_c1", "rq_ns", "beauty", "mlp", "kmeans", "gumbel", "tokenizer", "beam",
+                             "dropin"]
     for w in which:
         globals()["g_" + w]()

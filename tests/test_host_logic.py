@@ -14,7 +14,6 @@ from oracle import rq_oracle as O
 from parity import load_golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 def test_gin_shim_parses_the_reference_config_dialect():
@@ -68,39 +67,55 @@ def test_shard_bounds_cover_everything():
             assert max(h - l for l, h in b) - min(h - l for l, h in b) <= 1
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "modules")), reason="reference tree not present (GPU box)")
-def test_dropin_makes_the_unmodified_reference_import_the_replacements():
-    import ref_harness
-    ref_harness.install_stubs()
+def test_dropin_makes_the_unmodified_reference_import_the_replacements(tmp_path):
+    """tests/golden/dropin.npz, read from the unmodified reference tree: its imports of the aliased modules
+    (file:module:name), its RqVae / SemanticIdTokenizer calls (file:class:positional count:keywords), and the shipped
+    Beauty checkpoint with its tensor payloads zeroed (pickle byte for byte)."""
+    import inspect
+    g = load_golden("dropin")
+    root = tmp_path / "reference"                    # the reference's package skeleton: `modules` is a regular package
+    (root / "modules").mkdir(parents=True)
+    (root / "modules" / "__init__.py").write_text("")
+    ckpt = tmp_path / "checkpoint_high_entropy.pt"
+    ckpt.write_bytes(g["checkpoint"].tobytes())
     sys.modules.pop("gin", None)                     # let dropin register its own shim
-    for k in [k for k in sys.modules if k.split(".")[0] in ("modules", "init", "distributions", "train_rqvae", "data")]:
+    for k in [k for k in sys.modules if k.split(".")[0] in ("modules", "init", "distributions")]:
         del sys.modules[k]
     from rq_vae_recommender_b200 import dropin
+    from rq_vae_recommender_b200.modules.tokenizer import semids as mine_semids
     import rq_vae_recommender_b200.modules.rqvae as mine
     try:
-        dropin.install(reference_root=REF, replace_tokenizer=False)
-        import train_rqvae                                   # the UNMODIFIED script
-        import modules.tokenizer.semids as ref_semids        # the UNMODIFIED tokenizer
-        assert train_rqvae.RqVae is mine.RqVae
-        assert ref_semids.RqVae is mine.RqVae
-        assert train_rqvae.__file__.startswith(REF) and ref_semids.__file__.startswith(REF)
+        aliased = dropin.install(reference_root=str(root))
+        seen = set()
+        for line in g["imports"]:
+            path, module, name = str(line).split(":")
+            if module not in aliased:                # imported from the reference tree untouched
+                continue
+            ns = {}
+            exec(f"from {module} import {name}", ns)     # the reference's own import statement
+            assert getattr(ns[name], "__module__", "").startswith("rq_vae_recommender_b200"), (path, module, name)
+            seen.add((path, module, name))
+        assert ("train_rqvae.py", "modules.rqvae", "RqVae") in seen
+        assert ("modules/tokenizer/semids.py", "modules.rqvae", "RqVae") in seen
+        # the reference's constructor calls bind to the replacement classes (the training script and its tokenizer)
+        classes = {"RqVae": mine.RqVae, "SemanticIdTokenizer": mine_semids.SemanticIdTokenizer}
+        for line in g["calls"]:
+            path, cls, n_pos, kws = str(line).split(":")
+            inspect.signature(classes[cls]).bind(*[None] * int(n_pos), **dict.fromkeys(kws.split(",")))
+        assert any(str(line).startswith("modules/tokenizer/semids.py:RqVae:") for line in g["calls"])
         # a shipped checkpoint: state dict keys line up and the pickled model_config resolves to the replacements
-        path = os.path.join(REF, "trained_models/rqvae_amazon_beauty/checkpoint_high_entropy.pt")
-        state = torch.load(path, map_location="cpu", weights_only=False)
+        state = torch.load(str(ckpt), map_location="cpu", weights_only=False)
         m = mine.RqVae(input_dim=768, embed_dim=32, hidden_dims=[512, 256, 128], codebook_size=256,
                        codebook_kmeans_init=False, n_layers=3, n_cat_features=0)
         m.load_state_dict(state["model"])
         pickled_self = state["model_config"].get("self")
         assert pickled_self is None or type(pickled_self).__module__.startswith("rq_vae_recommender_b200")
-        tok = ref_semids.SemanticIdTokenizer(input_dim=768, output_dim=32, hidden_dims=[512, 256, 128], codebook_size=256,
-                                             n_layers=3, n_cat_feats=0)
-        assert type(tok.rq_vae) is mine.RqVae
     finally:
         dropin.uninstall()
-        for k in [k for k in sys.modules if k.split(".")[0] in ("train_rqvae", "modules", "data", "init", "distributions", "evaluate")]:
+        for k in [k for k in sys.modules if k.split(".")[0] in ("modules", "init", "distributions")]:
             del sys.modules[k]
-        if REF in sys.path:
-            sys.path.remove(REF)
+        if str(root) in sys.path:
+            sys.path.remove(str(root))
 
 
 # ------------------------------------------------------------------ world_size = 2 over gloo, kernels injected (CPU)
@@ -222,14 +237,15 @@ def test_forward_traces_to_one_graph_of_custom_operators(mode_name, train):
     assert names == {"rqb200.mlp_fwd.default", "rqb200.l2norm_fwd.default", "rqb200.count_unique_id_tuples.default", level}, names
 
 
-def test_bench_reference_arm_contract():
-    """`bench.py --impl reference` (the driver's reference arm) prints ONE JSON line with the contract's keys: the CPU port of the
-    reference path on this host's cores, same metric / unit / workload string as the GPU arm, zero copy bytes."""
+def test_bench_reference_arm_contract(tmp_path):
+    """`bench.py --impl reference` prints ONE JSON line with the keys of the GPU arm's line: the CPU port of the
+    reference path on this host's cores, same metric / unit / workload string as the GPU arm, zero copy bytes.  With
+    --dump-outputs it writes the last step's ids, which are the oracle's ids of the seeded batch."""
     import json
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1"],
-                         capture_output=True, text=True, timeout=600, cwd=root)
+    res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                          "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, timeout=600, cwd=root)
     assert res.returncode == 0, res.stderr[-2000:]
     lines = [l for l in res.stdout.strip().splitlines() if l.startswith("{")]
     assert len(lines) == 1
@@ -238,6 +254,12 @@ def test_bench_reference_arm_contract():
     assert d["higher_is_better"] is True and d["value"] > 0 and d["n_gpus"] == 1
     assert "65536x768" in d["config"]["workload"] and d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"] == {"value": d["value"], "unit": "items/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+    import bench
+    from parity import assert_ids_match
+    ids = np.load(tmp_path / "dump" / "ids.npy")
+    assert ids.dtype == np.float32 and ids.shape == (bench.N_ITEMS, bench.L)
+    x, cbs = bench.make_problem(8192)                     # the codebooks are drawn from the first 8192 rows
+    assert_ids_match(ids[:512].astype(np.int64), O.rq_tokenize(x[:512], cbs), x[:512], cbs)
 
 
 @pytest.mark.parametrize("kw", [dict(codebook_sim_vq=True), dict(codebook_normalize=True),

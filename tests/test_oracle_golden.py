@@ -29,6 +29,7 @@ def test_quantize_eval(tag):
     same = o.ids == g[f"{tag}_eval_ids"]
     assert rel_err(o.loss[same], g[f"{tag}_eval_loss"][same]) < TOL
     assert rel_err(o.embeddings[:keep][same[:keep]], g[f"{tag}_eval_emb"][same[:keep]]) < TOL
+    assert rel_err(o.embeddings.astype(np.float64).sum(1)[same], g[f"{tag}_eval_emb_rowsum"][same]) < TOL
 
 
 @pytest.mark.parametrize("tag", ["c1", "d32", "d768"])
@@ -42,6 +43,7 @@ def test_quantize_train_fwd_bwd(tag, mname):
     assert same.mean() > 0.999
     assert rel_err(o.loss[same], g[f"{tag}_{mname}_loss"][same]) < TOL
     assert rel_err(o.embeddings[:keep][same[:keep]], g[f"{tag}_{mname}_emb"][same[:keep]]) < 2e-5
+    assert rel_err(o.embeddings.astype(np.float64).sum(1)[same], g[f"{tag}_{mname}_emb_rowsum"][same]) < 2e-5
     gx, gc = O.quantize_backward(MODE[mname], x, cb, g[f"{tag}_{mname}_ids"].astype(np.int64), g_out, g_loss,
                                  BETA, T, u)
     # the gumbel softmax at T=0.2 amplifies fp32 rounding of dist by 1/T before exp(): looser there
