@@ -232,7 +232,7 @@ extern "C" int rqb200_tokenize_tc_run(const float* x, int64_t ldx, int B, const 
   const bool trace = want_trace && stats;       // tracing: the caller passes >= 4096 ints (tools/tc_native_check.cu)
   // Tile shape: 96-row CTAs move a third fewer codebook bytes and hand-offs per row and win once every CTA pair has several
   // tiles (12 101 rows: 0.041 vs 0.052 ms; 84 000: 0.193 vs 0.204); 64-row CTAs have the shorter pipeline and win below that
-  // (5 000 x 256: 0.053 vs 0.072 ms).  Both return identical ids (profiles/r2_tcx_shapes.txt).
+  // (5 000 x 256: 0.053 vs 0.072 ms).  Both return identical ids (tests/test_gpu_tc_variants.py).
   static const int force = []() { const char* e = getenv("RQB200_TC_ROWS"); return e ? atoi(e) : 0; }();
   const bool big = force ? force == 96 : (int64_t)B > 128ll * (sm_count / 2);     // more than one 64-row tile per CTA
   return big ? tcx_run_r96(x, ldx, B, state, D, L, ids, stats, sm_count, trace, st)

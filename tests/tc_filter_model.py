@@ -175,6 +175,22 @@ def adversarial_problem(kind: str, D: int = 768, K: int = 256, L: int = 1, n: in
             cb = base[rs.randint(0, 8, K)] * (1 + 3e-4 * rs.randn(K, 1))
             cbs.append(cb.astype(np.float32))
         return x, cbs
+    if kind == "opposite_rounding":
+        # x exact in fp16 (ex = 0) and, per row, two codes parallel to it whose fp16 roundings go opposite ways by 0.49 ulp per
+        # element: the scores move the truly closer code B up and the other code A down by ~eps each, so B stays a candidate
+        # only under the full 2 eps margin (B - A is 1.5e-4 in half-distance: far above fp32 noise and the near-tie tolerance).
+        # Row i follows sign pattern p = i % 64 with codes p and 128 + p, one in each CTA's half of the 256 codes; which of the
+        # two is B alternates with p.
+        a, ulp = 0.046875, 2.0 ** -15                  # 1.5 * 2^-5 is exact in fp16; ulp of its binade
+        pats = np.where(rs.rand(64, D) < 0.5, -1.0, 1.0)
+        x = (pats[np.arange(n) % 64] * a).astype(np.float32)
+        cb = (1e-3 * rs.randn(K, D)).astype(np.float32)
+        for p in range(64):
+            ib, ia = (p, 128 + p) if p % 2 == 0 else (128 + p, p)
+            cb[ib] = pats[p] * (a + 0.49 * ulp)        # rounds down to a
+            cb[ia] = pats[p] * (a - 20.49 * ulp)       # rounds up to a - 20 ulp
+        cbs = [cb] + [(1e-3 * rs.randn(K, D)).astype(np.float32) for _ in range(L - 1)]
+        return x, cbs
     if kind == "tiny_and_huge":
         # rows spanning fp16 subnormal .. overflow scales
         base = rs.randn(n, D)
@@ -187,4 +203,4 @@ def adversarial_problem(kind: str, D: int = 768, K: int = 256, L: int = 1, n: in
     raise ValueError(kind)
 
 
-ADVERSARIAL_KINDS = ["judge_r1", "sign_biased", "equal_magnitude", "code_parallel", "tiny_and_huge"]
+ADVERSARIAL_KINDS = ["judge_r1", "sign_biased", "equal_magnitude", "code_parallel", "tiny_and_huge", "opposite_rounding"]
